@@ -35,9 +35,11 @@ import subprocess
 import sys
 import tempfile
 import time
+import zlib
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 from speedseq_b200 import capi  # noqa: E402  (ctypes bindings of the product's C-ABI; no compute)
@@ -46,6 +48,10 @@ GENOME_LEN = 1000000000  # the largest round size the GPU index builder handles 
 READ_LEN = 150
 SB = dict(exclude_dups=1, add_mate_tags=1, max_split_count=2, min_non_overlap=20)  # bin/speedseq:439 with its defaults (:241-243)
 SB_ARGS = ["--excludeDups", "--addMateTags", "--maxSplitCount", "2", "--minNonOverlap", "20"]
+CONTIGS = ["chrS%d" % (i + 1) for i in range(8)]
+DUMP_PAIRS = 65536  # read pairs whose main-stream records --dump-outputs writes: ~11 MB at the default workload
+DUMP_SIDE_RECORDS = 131072  # splitter / discordant records beyond this many are sampled (90 k discordants at the default workload)
+DUMP_MAX_BYTES = 64 << 20
 
 
 # ------------------------------------------------------------------------------------ data ----
@@ -148,7 +154,7 @@ def ensure_reference(cache, genome_len, builder):
     if not os.path.exists(gnpy):
         g = synth_genome(genome_len, 20)
         bounds = np.linspace(0, genome_len, 9).astype(np.int64)
-        write_fasta(fa, g, ["chrS%d" % (i + 1) for i in range(8)], bounds)
+        write_fasta(fa, g, CONTIGS, bounds)
         np.save(gnpy, g)
         sys.stderr.write("[bench] synthetic genome of %d bp written in %.1f s\n" % (genome_len, time.time() - t0))
     if not all(os.path.exists(fa + e) for e in (".bwt", ".sa", ".pac", ".ann", ".amb")):
@@ -205,6 +211,55 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+class OutputDump:
+    """--dump-outputs: the SAM text of one step as float64 arrays, so that two builds can be compared output for output.
+    The three streams (0 main, 1 splitters, 2 discordants) are taken over all batches in input order:
+      summary.npy  [3, 3]: per stream [records, bytes, CRC-32 of the text]
+      records.npy  [n, 11]: one row per record: stream, pair id, FLAG, RNAME, POS, MAPQ, CRC-32 of CIGAR, RNEXT, PNEXT, TLEN,
+                   CRC-32 of the whole line (contigs numbered from 0, '*' = -1).  Main stream: every record of a fixed, seeded
+                   sample of DUMP_PAIRS read pairs.  Side streams: every record (they are small; a few per million reads are
+                   splitters, which no pair sample would reliably hit), a fixed, seeded sample of DUMP_SIDE_RECORDS beyond that."""
+
+    def __init__(self, pair_ids):
+        rng = np.random.default_rng(7)
+        self.keep = np.sort(rng.choice(pair_ids, min(DUMP_PAIRS, len(pair_ids)), replace=False))
+        self.summary = np.zeros((3, 3))
+        self.rows = [[] for _ in range(3)]
+        self.ctg = {c.encode(): i for i, c in enumerate(CONTIGS)}
+        self.ctg[b"*"] = -1
+
+    def add(self, k, text):
+        """text: one batch's stream k, any buffer (read in place, not copied)"""
+        buf = np.frombuffer(text, np.uint8)
+        ends = np.flatnonzero(buf == 10)
+        starts = np.concatenate(([0], ends[:-1] + 1)) if len(ends) else ends
+        self.summary[k] += [len(ends), len(buf), 0]
+        self.summary[k, 2] = zlib.crc32(buf, int(self.summary[k, 2]))
+        if k == 0:
+            ids = (buf[starts[:, None] + np.arange(1, 10)].astype(np.int64) - 48) @ 10 ** np.arange(8, -1, -1, dtype=np.int64)  # QNAME p%09d
+            sel = np.isin(ids, self.keep)
+            starts, ends = starts[sel], ends[sel]
+        for s, e in zip(starts, ends):
+            line = buf[s:e].tobytes()
+            f = line.split(b"\t")
+            rname = self.ctg[f[2]]
+            self.rows[k].append((k, int(f[0][1:]), int(f[1]), rname, int(f[3]), int(f[4]), zlib.crc32(f[5]), rname if f[6] == b"=" else self.ctg[f[6]],
+                                 int(f[7]), int(f[8]), zlib.crc32(line)))
+
+    def write(self, d):
+        rows = [np.array(r, np.float64).reshape(-1, 11) for r in self.rows]
+        for k in (1, 2):
+            if len(rows[k]) > DUMP_SIDE_RECORDS:
+                rows[k] = rows[k][np.sort(np.random.default_rng(7 + k).choice(len(rows[k]), DUMP_SIDE_RECORDS, replace=False))]
+        arrays = {"summary": self.summary, "records": np.concatenate(rows)}
+        total = sum(a.nbytes for a in arrays.values())
+        if total > DUMP_MAX_BYTES:
+            raise SystemExit("bench.py: --dump-outputs would write %d bytes, more than %d" % (total, DUMP_MAX_BYTES))
+        os.makedirs(d, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(d, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------- CPU arm ----
 def oracle_lib():
     sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -244,7 +299,9 @@ def main():
     ap.add_argument("--reads", type=int, default=10_000_000)
     ap.add_argument("--batch", type=int, default=2_000_000)
     ap.add_argument("--genome-len", type=int, default=int(os.environ.get("SSQ_BENCH_GENOME", GENOME_LEN)))
-    ap.add_argument("--cache", default=os.environ.get("SSQ_BENCH_CACHE", os.path.join(ROOT, "data_cache")))
+    ap.add_argument("--cache", default=os.environ.get("SSQ_BENCH_CACHE", os.path.join(tempfile.gettempdir(), "ssq_bench_cache_%d" % os.getuid())),
+                    help="directory for the synthetic reference and its index (reused by later runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the SAM records of the last step as .npy arrays (class OutputDump)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample", type=int, default=0, help="reads in the CPU-arm sample (0: sized for ~15 s)")
     ap.add_argument("--streams", type=int, default=int(os.environ.get("SSQ_BENCH_STREAMS", "5")), help="host threads / CUDA streams that drive batches concurrently")
@@ -279,10 +336,15 @@ def main():
         n_run = int(min(n_s, max(n_try, r * 8.0))) & ~1  # ~8 s per step
         for s in range(a.warmup + a.steps):
             n = n_run if s >= a.warmup else min(n_run, 20000)
-            r, dt, _, parts = cpu_arm(T, o, oidx, fa, b0, n, ncores)
+            r, dt, streams, parts = cpu_arm(T, o, oidx, fa, b0, n, ncores)
             if s >= a.warmup:
                 rates.append(r)
                 desc = "%d reads per step (a batch of the same generator as the workload), bwa-mem port on %d threads %.1f s + samblaster port (1 thread, like the reference) %.1f s" % (n, ncores, parts[0], parts[1])
+        if a.dump_outputs:
+            dump = OutputDump(np.arange(n // 2))
+            for k in range(3):
+                dump.add(k, streams[k])
+            dump.write(a.dump_outputs)
         v = float(np.mean(rates))
         print(json.dumps({"impl": "reference", "metric": metric, "value": v, "unit": "reads/s", "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup,
                           "ms_per_step": 1000.0 * n_run / v, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "int32", "data": "synthetic",
@@ -387,6 +449,14 @@ def main():
     barrier()
     ms_total = span_ms(ev)
     clocks = clk.stop()
+    if a.dump_outputs and rank == 0:  # what the last timed step left in each aligner: rank 0's batches
+        dump = OutputDump(np.concatenate([(b * world + rank) * (a.batch // 2) + np.arange(a.batch // 2) for b in range(nb)]))
+        sam = capi.Sam()
+        for al in aligners:
+            s.ck(L.ssq_aligner_fetch(al, C.byref(sam)), "ssq_aligner_fetch")
+            for k in range(3):
+                dump.add(k, (C.c_char * sam.len[k]).from_address(sam.text[k]))
+        dump.write(a.dump_outputs)
     # ---- per-stage statistics: one extra step, batches one after the other so that stage durations are not stretched by overlap ----
     STAGES = ["upload", "seed_chain_extend", "sort_dedup_patch", "insert_size_stats", "mate_rescue", "pair_mapq_plan", "cigar_nm_md", "samblaster_dupset", "sam_text", "fetch",
               "k_smem", "k_sa", "k_chain", "k_extend", "k_select"]

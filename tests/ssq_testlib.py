@@ -20,6 +20,12 @@ from speedseq_b200.capi import SMEM_DT, SEED_DT, SWTASK_DT, SWRES_DT, REG_DT, DU
 ODUPSIG_DT = np.dtype([("pos1", "<u8"), ("pos2", "<u8"), ("strand1", "u1"), ("strand2", "u1"), ("valid", "u1")], align=True)
 
 
+def gpu_visible():
+    """a CUDA device is usable from this process, as the CUDA runtime sees it (a process's GPU need not be /dev/nvidia0)"""
+    import torch
+    return torch.cuda.is_available()
+
+
 def build_oracle():
     subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle")])
 

@@ -37,7 +37,7 @@ def test_default_options_match_oracle(oracle):
     assert C.sizeof(s.opts) == 30 * 4
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="box has a GPU")
+@pytest.mark.skipif(T.gpu_visible(), reason="box has a GPU")
 def test_no_cpu_fallback_without_gpu(ex_index):
     s = T.SSQ()
     h = C.c_void_p()

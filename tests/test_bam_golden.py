@@ -3,6 +3,8 @@ against what the REFERENCE'S OWN TOOL makes of the oracle's SAM text: tests/gold
 /root/reference/src/sambamba v0.5.9 (`view -S -f bam -l 0 | sort`, the commands of bin/speedseq:440-448) — see
 tests/golden/make_bam_golden.py.  CPU: the encoder bodies through tests/hostsim.  GPU: the kernels through ssq_aligner_fetch_bam."""
 import gzip
+import hashlib
+import json
 import os
 
 import pytest
@@ -110,18 +112,32 @@ def test_bam_records_match_sambamba_gpu(ssq, ex_index, ex_reads):
     ssq.index_free(h)
 
 
-def test_bgzf_framing_roundtrip_and_sambamba_reads_it(ssq_lib_cpu, oracle, hostsim, ex_index, ex_reads, tmp_path):
-    """ssq_bgzf_compress (host, zlib): members of at most 64 KiB with the BC extra field and the EOF marker; python's gzip and, where the
-    reference checkout is present (this container, not the GPU box), the reference's sambamba read the resulting .bam back"""
-    import ctypes as C
+def sambamba_golden(name):
+    """what the reference's sambamba v0.5.9 made of a BAM file a test writes (tests/golden/make_sambamba_golden.py)"""
+    return json.load(open(os.path.join(T.GOLDEN, "sambamba_reads.json")))[name]
+
+
+def sha256(b):
+    return hashlib.sha256(b).hexdigest()
+
+
+def example_bam(oracle, hostsim, ex_index, ex_reads):
+    """(uncompressed BAM of the example reads' main records, the oracle pipeline's SAM text of them)"""
     import struct
-    import subprocess
-    L = ssq_lib_cpu
     idx = oracle.load(ex_index)
     names, seqs, quals = ex_reads
     txt, bams = hostsim.pipe_bam(idx, names, seqs, quals, 0, b"NA12878", 1, (1, 1, 2, 20, 0))
     hdr_text = b"@HD\tVN:1.3\tSO:coordinate\n@SQ\tSN:20_slice\tLN:321635\n@RG\tID:NA12878\tSM:NA12878\tLB:lib1\n"
-    raw = b"BAM\x01" + struct.pack("<i", len(hdr_text)) + hdr_text + struct.pack("<i", 1) + struct.pack("<i", 9) + b"20_slice\x00" + struct.pack("<i", 321635) + bams[0]
+    return b"BAM\x01" + struct.pack("<i", len(hdr_text)) + hdr_text + struct.pack("<i", 1) + struct.pack("<i", 9) + b"20_slice\x00" + struct.pack("<i", 321635) + bams[0], txt[0]
+
+
+def test_bgzf_framing_roundtrip_and_sambamba_reads_it(ssq_lib_cpu, oracle, hostsim, ex_index, ex_reads):
+    """ssq_bgzf_compress (host, zlib): members of at most 64 KiB with the BC extra field and the EOF marker; python's gzip reads the
+    resulting .bam back, and the reference's sambamba read the same BAM as the oracle pipeline's records (golden)"""
+    import ctypes as C
+    import struct
+    L = ssq_lib_cpu
+    raw, main_text = example_bam(oracle, hostsim, ex_index, ex_reads)
     for level in (0, 1, 6):
         out, n = C.c_void_p(), C.c_size_t(0)
         assert L.ssq_bgzf_compress(raw, C.c_size_t(len(raw)), C.c_int(level), C.c_int(1), C.byref(out), C.byref(n)) == 0
@@ -136,15 +152,12 @@ def test_bgzf_framing_roundtrip_and_sambamba_reads_it(ssq_lib_cpu, oracle, hosts
             p += bsize; nb += 1
         assert p == len(comp) and nb == (len(raw) + 0xff00 - 1) // 0xff00 + 1
         assert comp.endswith(bytes([0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 0x42, 0x43, 2, 0, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0]))
-    sb = "/root/reference/src/sambamba"
-    if os.path.exists(sb):
-        bam = str(tmp_path / "x.bam")
-        open(bam, "wb").write(comp)
-        view = subprocess.run([sb, "view", bam], check=True, stdout=subprocess.PIPE, stderr=subprocess.DEVNULL).stdout.decode()
-        assert view.count("\n") == txt[0].count("\n")
-        # sambamba's text of our records == the oracle pipeline's SAM records, re-ordered by coordinate (stable)
-        key = lambda l: (1 << 40 if l.split("\t")[2] == "*" else 0, int(l.split("\t")[3]), (int(l.split("\t")[1]) >> 4) & 1)
-        assert view.splitlines() == sorted(txt[0].splitlines(), key=key)
+    # sambamba's text of these bytes == the oracle pipeline's SAM records, re-ordered by coordinate (stable)
+    want = sambamba_golden("bgzf_example")
+    assert sha256(raw) == want["bam_sha256"]
+    key = lambda l: (1 << 40 if l.split("\t")[2] == "*" else 0, int(l.split("\t")[3]), (int(l.split("\t")[1]) >> 4) & 1)
+    view = sorted(main_text.splitlines(), key=key)
+    assert len(view) == want["view_lines"] and sha256("".join(l + "\n" for l in view).encode()) == want["view_sha256"]
 
 
 def test_header_rewrite_matches_sambamba(ssq_lib_cpu):
@@ -191,14 +204,9 @@ def _bam_file(path):
     return text, refs, d[q:]
 
 
-def test_sambamba_shim_merges_the_run_stream(ssq_lib_cpu, oracle, hostsim, syn_index, tmp_path):
-    """BAM mode of the shims (ssq_fuse.h): header text + marker + one frame per batch through `sambamba view -S -f bam -l 0 /dev/stdin |
-    sambamba sort ... -o out.bam /dev/stdin` as speedseq:440-441 calls them.  The file's records must be the reference sambamba's
-    (golden syn3), its header the rewritten one, with and without spilling to --tmpdir, for any thread count."""
-    import ctypes as C
+def shim_run_stream(oracle, hostsim, syn_index):
+    """(SAM header, what the `bwa` shim writes in BAM mode for the synthetic reads as a run of three batches: header, marker, frames)"""
     import struct
-    import subprocess
-    shim = os.path.join(T.ROOT, "speedseq_b200", "bin", "sambamba")
     idx = oracle.load(syn_index[0])
     names, seqs, quals = syn_reads(syn_index)
     cuts = [0, 1000, 2100, len(names)]
@@ -208,6 +216,17 @@ def test_sambamba_shim_merges_the_run_stream(ssq_lib_cpu, oracle, hostsim, syn_i
     for k, (a, b) in enumerate(zip(cuts, cuts[1:])):
         txt, bams = hostsim.pipe_bam(idx, names[a:b], seqs[a:b], quals[a:b], a, b"NA12878", 1, (1, 1, 2, 20, 0), reset=1 if k == 0 else 0)
         stream += b"SSQFRAME" + struct.pack("<QQ", 3, len(bams[0])) + bams[0]
+    return hdr, stream
+
+
+def test_sambamba_shim_merges_the_run_stream(ssq_lib_cpu, oracle, hostsim, syn_index, tmp_path):
+    """BAM mode of the shims (ssq_fuse.h): header text + marker + one frame per batch through `sambamba view -S -f bam -l 0 /dev/stdin |
+    sambamba sort ... -o out.bam /dev/stdin` as speedseq:440-441 calls them.  The file's records must be the reference sambamba's
+    (golden syn3), its header the rewritten one, with and without spilling to --tmpdir, for any thread count."""
+    import ctypes as C
+    import subprocess
+    shim = os.path.join(T.ROOT, "speedseq_b200", "bin", "sambamba")
+    hdr, stream = shim_run_stream(oracle, hostsim, syn_index)
     L = ssq_lib_cpu
     L.ssq_bam_header_text.argtypes = [C.c_char_p, C.c_int, C.c_void_p]
     out = C.c_void_p()
@@ -227,17 +246,17 @@ def test_sambamba_shim_merges_the_run_stream(ssq_lib_cpu, oracle, hostsim, syn_i
         files.append(open(o, "rb").read())
     assert files[0] == files[1]  # block boundaries do not depend on threads or spills
     assert not [f for f in os.listdir(tmp_path) if f.endswith(".run")]
-    real = next((p for p in ("/root/reference/src/sambamba", os.path.join(T.ROOT, "oracle", "_ref", "stage", "src", "sambamba")) if os.access(p, os.X_OK)), None)
-    if real:  # the reference's sambamba reads the file, and foreign input goes through the shim to it unchanged
-        n = subprocess.run([real, "view", "-c", str(tmp_path / "plain.bam")], stdout=subprocess.PIPE, check=True).stdout
-        assert int(n) == len(split_records(golden("main", "syn3")))
-        sam = hdr + b"r1\t4\t*\t0\t0\t*\t*\t0\t0\tACGT\tIIII\n"
-        a = subprocess.run([real, "view", "-S", "-f", "bam", "-l", "0", "/dev/stdin"], input=sam, stdout=subprocess.PIPE, check=True).stdout
-        b = subprocess.run([shim, "view", "-S", "-f", "bam", "-l", "0", "/dev/stdin"], input=sam, stdout=subprocess.PIPE, check=True, env=dict(os.environ, SSQ_SAMBAMBA_REAL=real)).stdout
-        assert a == b and a[:2] == b"\x1f\x8b"
-        o2 = str(tmp_path / "foreign.bam")
-        subprocess.run([shim, "sort", "-t", "2", "-m", "1G", "--tmpdir=" + str(tmp_path), "-o", o2, "/dev/stdin"], input=b, check=True, env=dict(os.environ, SSQ_SAMBAMBA_REAL=real))
-        assert int(subprocess.run([real, "view", "-c", o2], stdout=subprocess.PIPE, check=True).stdout) == 1
+    # the reference's sambamba read the file's BAM content and counted every record (golden)
+    want = sambamba_golden("shim_sort")
+    assert sha256(gzip.decompress(files[0])) == want["bam_sha256"] and want["records"] == len(split_records(golden("main", "syn3")))
+    # foreign input goes through the shim to the real sambamba unchanged: arguments and bytes, seen by a stand-in that echoes both
+    real = tmp_path / "sambamba.real"
+    real.write_text('#!/bin/sh\nprintf "%s\\n" "$*"\nexec cat\n')
+    real.chmod(0o755)
+    sam = hdr + b"r1\t4\t*\t0\t0\t*\t*\t0\t0\tACGT\tIIII\n"
+    for argv in (["view", "-S", "-f", "bam", "-l", "0", "/dev/stdin"], ["sort", "-t", "2", "-m", "1G", "--tmpdir=" + str(tmp_path), "-o", str(tmp_path / "foreign.bam"), "/dev/stdin"]):
+        b = subprocess.run([shim] + argv, input=sam, stdout=subprocess.PIPE, check=True, timeout=60, env=dict(os.environ, SSQ_SAMBAMBA_REAL=str(real))).stdout
+        assert b == (" ".join(argv) + "\n").encode() + sam, argv
 
 
 def test_bam_mode_chain_of_the_three_shims_cpu(oracle, hostsim, ex_index, ex_reads, tmp_path):

@@ -1,7 +1,8 @@
 """BASELINE config 1 plumbing on the CPU: the reference's UNMODIFIED bin/speedseq with a private config whose $BWA / $SAMBLASTER are the
 oracle CLI (argv-identical to the shims) — once with the reference's sambamba, once with `SAMBAMBA=` the repo's sambamba shim, which
 has to hand every call of the script (view / sort of plain SAM and BAM, index) through to the real one.  Same three BAMs both ways.
-Runs only where the reference checkout exists (this build container); the GPU-side runs are profiles/r02_config1_unmodified_speedseq.log."""
+The script, the binary and the example data are the reference's own and are not part of this repository: the test runs where build()
+staged them under oracle/_ref/stage (tools/stage_config1.sh) and skips elsewhere; the GPU-side runs are profiles/r02_config1_unmodified_speedseq.log."""
 import os
 import subprocess
 
@@ -9,8 +10,8 @@ import pytest
 
 import ssq_testlib as T
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not (os.path.exists(REF + "/bin/speedseq") and os.access(REF + "/src/sambamba", os.X_OK)), reason="no reference checkout on this box")
+REF = os.path.join(T.ROOT, "oracle", "_ref", "stage")
+pytestmark = pytest.mark.skipif(not (os.path.exists(REF + "/bin/speedseq") and os.access(REF + "/src/sambamba", os.X_OK)), reason="the reference's speedseq script and sambamba are not staged under oracle/_ref/stage")
 
 
 def test_unmodified_speedseq_runs_with_the_sambamba_shim_in_front_of_the_real_one(tmp_path):

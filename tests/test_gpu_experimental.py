@@ -1,14 +1,11 @@
-"""GPU parity of the seeding paths that are implemented and CPU-validated (tests/hostsim) but have not been measured / verified on a
-GPU yet: the lean backward kernel (SSQ_SMEM_VARIANT=4), the k-mer jump-start table (SSQ_KMER_K) and the split path's pool-overflow
-retry.  Skipped unless SSQ_TEST_EXPERIMENTAL=1 — run them first thing when a GPU is available (tools/round2_first_runs.sh)."""
-import os
-
+"""GPU parity of the seeding paths that are not the default: the lean backward kernel (SSQ_SMEM_VARIANT=4), the k-mer jump-start
+table (SSQ_KMER_K) and the split path's pool-overflow retry."""
 import numpy as np
 import pytest
 
 import ssq_testlib as T
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(os.environ.get("SSQ_TEST_EXPERIMENTAL") != "1", reason="experimental seeding variants: set SSQ_TEST_EXPERIMENTAL=1")]
+pytestmark = pytest.mark.gpu
 
 
 def _reads(syn_index, n=1500, seed=41):

@@ -56,7 +56,7 @@ def test_host_index_equals_oracle_on_synthetic_genomes(ssq_lib_cpu, oracle, tmp_
 
 def test_small_reference_still_needs_the_gpu(ssq_lib_cpu, tmp_path, monkeypatch):
     """without the knob a reference the device sort holds goes to the device: on a box without a GPU that is an error, not a silent CPU build"""
-    if os.path.exists("/dev/nvidia0"):
+    if T.gpu_visible():
         pytest.skip("a GPU is present")
     monkeypatch.delenv("SSQ_INDEX_HOST", raising=False)
     fa = str(tmp_path / "ex.fa")
