@@ -87,7 +87,9 @@ int ssq_smem_batch(const ssq_index_t *idx, const ssq_opts_t *opt, int n_reads, c
 int ssq_sa_lookup_batch(const ssq_index_t *idx, uint64_t n, const uint64_t *rows, uint64_t *pos);
 
 /* Banded affine-gap seed extension.  Replaces upstream ksw_extend2() as called from
- * mem_chain2aln() (speedseq:438).  Sequences are one byte per base in qbuf/tbuf. */
+ * mem_chain2aln() (speedseq:438).  Sequences are one byte per base in qbuf/tbuf.
+ * Each task needs 1 <= qlen <= SSQ_MAX_READ_LEN, h0 >= 1 and h0 + qlen * opt->a <= 65535: the DP row keeps H and E in
+ * 16 bits each, so a larger possible score fails the call with SSQ_EINVAL (the pipeline's own extensions stay far below). */
 typedef struct { uint64_t q_off, t_off; int32_t qlen, tlen, h0, w, end_bonus, zdrop; } ssq_sw_task_t;
 typedef struct { int32_t score, qle, tle, gtle, gscore, max_off; } ssq_sw_result_t;
 int ssq_sw_extend_batch(const ssq_opts_t *opt, int device, uint64_t n, const ssq_sw_task_t *tasks,

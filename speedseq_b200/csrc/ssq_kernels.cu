@@ -2038,6 +2038,11 @@ extern "C" int ssq_sw_extend_batch(const ssq_opts_t *opt, int device, uint64_t n
 		if (tasks[i].qlen < 1 || tasks[i].qlen > SSQ_MAX_READ_LEN || tasks[i].h0 < 1 || tasks[i].q_off + tasks[i].qlen > qbuf_len || tasks[i].t_off + tasks[i].tlen > tbuf_len) {
 			ssq_set_error("ssq_sw_extend_batch: task %llu out of range", (unsigned long long)i); return SSQ_EINVAL;
 		}
+		if ((long long)tasks[i].h0 + (long long)tasks[i].qlen * opt->a > 65535) { // the DP row keeps H and E in 16 bits each (sw_extend_impl)
+			ssq_set_error("ssq_sw_extend_batch: task %llu: h0 + qlen * a = %lld exceeds 65535, the largest score the DP row holds", (unsigned long long)i,
+			              (long long)tasks[i].h0 + (long long)tasks[i].qlen * opt->a);
+			return SSQ_EINVAL;
+		}
 		if (tasks[i].qlen > qmax) qmax = tasks[i].qlen;
 	}
 	DBuf dt, dq, dtb, dout;

@@ -265,4 +265,8 @@ def test_sw_local_striped_order(ssq, oracle):
         ref[i] = (r.score, r.te, r.qe, r.score2, r.te2, r.tb, r.qb)
     bad = np.nonzero(got != ref)[0]
     assert len(bad) == 0, (bad[:5], got[bad[:5]], ref[bad[:5]], tasks[bad[:5]])
-    assert (ref["score"] >= 19).sum() > 500 and (ref["score2"] >= 19).sum() > 50 and (ref["score"] == 255).sum() >= 0
+    assert (ref["score"] >= 19).sum() > 500 and (ref["score2"] >= 19).sum() > 50
+    # both modes found hits, byte mode up to scores near its 255 ceiling (saturation itself: test_gpu_edges.py::test_sw_local_grid)
+    byte = (tasks["xtra"] & 0x10000) != 0
+    assert (byte & (ref["score"] >= 19)).sum() > 600 and (byte & (ref["score"] >= 200)).sum() > 50 and (~byte & (ref["score"] >= 19)).sum() > 50
+    assert (ref["tb"] >= 0).sum() > 600
